@@ -3,6 +3,7 @@
 
   python bench.py --gpus N --steps K --warmup W            (N>1: launched under torchrun, one rank per GPU)
   python bench.py --impl reference --gpus N --steps K --warmup W
+  python bench.py --gpus 1 --steps K --warmup W --dump-outputs DIR    (also writes the last timed step's result rows)
 
 Workload (BASELINE.json configs[1]): Q1's scan + filter + GROUP BY (l_returnflag, l_linestatus) with its
 8 aggregates (no ORDER BY) over a 10^8-row synthetic lineitem heap relation (16 columns, 32 KB pages,
@@ -358,6 +359,23 @@ def q1_combine(parts):
     return out
 
 
+Q1_COLUMNS = ("l_returnflag", "l_linestatus", "sum_qty", "sum_base_price", "sum_disc_price", "sum_charge", "avg_qty", "avg_price",
+              "avg_disc", "count_order")
+
+
+def dump_q1_rows(rows, outdir):
+    """Executor.rows() of the Q1 plan -> outdir/<output column>.npy, float64, one entry per group in (l_returnflag, l_linestatus)
+    order, since a hash aggregate hands its groups up in no fixed order.  The two keys are stored as their character codes, the
+    float8 aggregates bit for bit, count(*) exactly (float64 holds integers up to 2^53).  So two builds, run with the same
+    arguments over the same seeded relation, can be compared column by column."""
+    groups = sorted((capi.unpack_str(v[0], ln[0]), capi.unpack_str(v[1], ln[1]), [b2f(v[2 + i]) for i in range(7)], int(v[9]))
+                    for v, nl, ty, ln in rows)
+    os.makedirs(outdir, exist_ok=True)
+    cols = [[ord(g[0]) for g in groups], [ord(g[1]) for g in groups]] + [[g[2][i] for g in groups] for i in range(7)] + [[g[3] for g in groups]]
+    for name, col in zip(Q1_COLUMNS, cols):
+        np.save(os.path.join(outdir, name + ".npy"), np.array(col, dtype=np.float64))
+
+
 def q1_compare(got, want, tol=1e-6):
     """-> parity dict; counts and keys bit-exact, float8 aggregates within tol relative"""
     ok = set(got) == set(want)
@@ -391,7 +409,11 @@ def main():
     ap.add_argument("--narrow-rows", type=float, default=1e9)
     ap.add_argument("--rjoin-rows", type=float, default=2e8, help="lineitem rows of the Redistribute-HashJoin, TOTAL over all GPUs")
     ap.add_argument("--rjoin-child", default=None, help=argparse.SUPPRESS)      # internal: see rjoin_in_children
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="write the result rows of the last timed step as DIR/<output column>.npy (float64)")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
     args.rows = int(args.rows)
     args.warmup = max(args.warmup, 3) if args.impl != "reference" else args.warmup
 
@@ -483,11 +505,17 @@ def main():
 
     scan_ms_tot, scan_launches = 0.0, 0
     last_rows = [0]
+    kept_rows = None
 
-    def step_resident():
-        nonlocal scan_ms_tot, scan_launches
+    def step_resident(keep=False):
+        """keep: hand the rows up as Python lists (kept_rows) instead of only counting them; 4 rows, microseconds"""
+        nonlocal scan_ms_tot, scan_launches, kept_rows
         x.rescan()
-        last_rows[0] = x.drain()
+        if keep:
+            kept_rows = x.rows()
+            last_rows[0] = len(kept_rows)
+        else:
+            last_rows[0] = x.drain()
         ms, k, _, _ = x.kernel_ms()
         scan_ms_tot += ms
         scan_launches += k
@@ -509,8 +537,8 @@ def main():
     barrier()
     l0 = eng.launch_count()
     eng.timer_start()
-    for _ in range(args.steps):
-        step_resident()
+    for i in range(args.steps):
+        step_resident(keep=args.dump_outputs is not None and i == args.steps - 1)
     ms = eng.timer_stop()
     barrier()
     launches = eng.launch_count() - l0
@@ -521,6 +549,8 @@ def main():
     scan_ms = scan_ms_tot / max(scan_launches, 1)
     variant = x.kernel_ms()[2]
     result_rows = last_rows[0]
+    if args.dump_outputs is not None and rank == 0:
+        dump_q1_rows(kept_rows, args.dump_outputs)
 
     # ---- end to end: pages start in host memory every step (same plan, the relation given as host pages) ----
     e2e = None

@@ -26,6 +26,10 @@
   mvcc_kat.json     the reference's tqual.o + transam.o: HeapTupleSatisfiesMVCC of tuple headers against snapshots and
                     transaction status tables (oracle/ref_build/refwrap_tqual.c)
   join_j1j2.json    J1_TBL / J2_TBL of sql/join.sql and the golden inner / left / right / full equi-join tables of expected/join.out
+  hash_random_kat.json  digests of the reference's hashes and routing of test_oracle_hash.py's 20000 random inputs
+  aocs_random_kat.json  digests of the column files the reference writes for test_oracle_aocs.py's random columns, and of
+                    what its reader returns for them
+  wire_kat.json     tuple chunks exchanged with the reference's tupser.o / tupchunklist.o in test_executor_wire.py
 """
 import ctypes as C
 import json
@@ -41,6 +45,7 @@ import numpy as np
 HERE = os.path.dirname(os.path.abspath(__file__))
 ROOT = os.path.dirname(os.path.dirname(HERE))
 sys.path.insert(0, ROOT)
+sys.path.insert(0, os.path.dirname(HERE))             # the tests whose random inputs some fixtures answer for
 from greengage_b200 import capi  # noqa: E402
 from oracle import pyoracle as po  # noqa: E402
 
@@ -671,6 +676,90 @@ def aocs_kat():
     print("aocs_kat.npz", len(names), "column files")
 
 
+def hash_random_kat():
+    """The reference's hash_any / hashint8 / cdbhash routing of the random inputs tests/test_oracle_hash.py draws
+    (random.Random(7)), as SHA-256 digests of each output sequence: 20000 cases in a few bytes."""
+    import test_oracle_hash as th
+    from test_oracle_aocs import sha256
+    out = {"cases": th.RANDOM_CASES}
+    for name, fn in (("hash_any", R.ref_hash_any), ("hashint8", R.ref_hashint8), ("route", R.ref_cdbhash_route)):
+        out[name] = sha256(th.random_hash_outputs(fn, name))
+    json.dump(out, open(os.path.join(HERE, "hash_random_kat.json"), "w"), indent=1)
+    print("hash_random_kat.json", out)
+
+
+def aocs_random_kat():
+    """Random column files the reference's own writer makes for tests/test_oracle_aocs.py's random inputs (np.random.default_rng(77),
+    32 KB blocks), and what its own reader returns for them, as SHA-256 digests: the files are megabytes, the digests are not."""
+    import test_oracle_aocs as ta
+    out = []
+    for name, nullfrac, a, vals, nulls in ta.random_columns():
+        f = po.aocs_write_column(a, vals, nulls, ref=True)
+        rv, rn, rf, rr = po.aocs_read_column(a, f, len(vals), ref=True)
+        out.append({"type": name, "nullfrac": nullfrac, "rows": len(vals), "file_bytes": int(f.size), "file": ta.sha256(f),
+                    "read": ta.sha256(rv, rn, rf, rr), "max_rows_per_block": int(rr.max())})
+    json.dump(out, open(os.path.join(HERE, "aocs_random_kat.json"), "w"), indent=1)
+    print("aocs_random_kat.json", len(out), "column files")
+
+
+def wire_kat():
+    """Tuple chunks across a Motion, as tests/test_executor_wire.py exchanges them with the reference's tupser.o / tupchunklist.o:
+      partial  the PARTIAL-stage Q1 rows of segment 0 as the product's GgExecSendTupleChunks writes them (two chunk sizes), and
+               what the reference's CvtChunksToTup reads from each tuple's chunks
+      senders  every segment's rows written by the reference's SerializeTuple, as a MemTuple and as a heap tuple"""
+    import tempfile
+    import test_executor_wire as tw
+    from greengage_b200 import executor as ex
+    L = tw.bind_mock(C.CDLL(tw.build_mock(tempfile.mkdtemp())))
+    old, ex._lib = ex._lib, L
+    eng = L.mock_engine()
+    # the PARTIAL Q1 row: two bpchar keys, four float8 sums, three float8[] {N, sumX, sumX2}, count
+    wire = [(1042, -1, 'i', 0), (1042, -1, 'i', 0)] + [(701, 8, 'd', 1)] * 4 + [(1022, -1, 'd', 0)] * 3 + [(20, 8, 'd', 1)]
+    attrs = (capi.gg_attr * len(wire))()
+    for i, (t, l, al, bv) in enumerate(wire):
+        attrs[i].atttypid, attrs[i].attlen, attrs[i].attalign, attrs[i].attbyval, attrs[i].atttypmod = t, l, ord(al), bv, -1
+    out = {"partial": {}, "senders": {"ref-memtuple": [], "ref-heap": []}}
+    for max_chunk in tw.PARTIAL_CHUNK_SIZES:
+        stream, n, rows = tw.partial_chunks(L, eng, 0, max_chunk)
+        read, pos = [], 0
+        for _ in rows:
+            end = pos                                   # one tuple's chunks: up to and including the WHOLE / PARTIAL_END chunk
+            while True:
+                size, typ = struct.unpack_from("<HH", stream, end)
+                end += 4 + size
+                if typ in (0, 3):
+                    break
+            vals, lens, nulls, sb = (C.c_int64 * 10)(), (C.c_int32 * 10)(), (C.c_uint8 * 10)(), (C.c_uint8 * 1024)()
+            form = R.ref_deserialize_tuple(10, attrs, stream[pos:end], end - pos, vals, lens, nulls, sb, 1024)
+            sbb = bytes(sb)
+            read.append({"form": form, "nulls": list(nulls),
+                         "keys": [sbb[vals[k]:vals[k] + lens[k]].decode() for k in range(2)],
+                         "sums": list(vals[2:6]), "count": vals[9],
+                         "arrays": [list(struct.unpack_from("<iiIii3q", sbb, vals[6 + k])) for k in range(3)],
+                         "array_lens": list(lens[6:9])})
+            pos = end
+        assert pos == len(stream) - 4
+        out["partial"][str(max_chunk)] = {"stream": stream.hex(), "read": read}
+    for form in out["senders"]:
+        for seg in range(tw.NSEG):
+            _, _, rows = tw.partial_chunks(L, eng, seg, 8124)
+            parts = []
+            for v, nl, ty, ln in rows:
+                keep = [C.create_string_buffer(capi.unpack_str(v[k], ln[k]).encode(), max(ln[k], 1)) for k in range(2)]
+                arrs = [C.create_string_buffer(struct.pack("<iiIii3q", 1, 0, 701, 3, 1, *v[6 + 3 * k:9 + 3 * k]), 44) for k in range(3)]
+                vals = (C.c_int64 * 10)(C.addressof(keep[0]), C.addressof(keep[1]), v[2], v[3], v[4], v[5],
+                                        C.addressof(arrs[0]), C.addressof(arrs[1]), C.addressof(arrs[2]), v[15])
+                lens = (C.c_int32 * 10)(ln[0], ln[1], 0, 0, 0, 0, 44, 44, 44, 0)
+                buf, nch = (C.c_uint8 * 4096)(), C.c_int32(0)
+                t = R.ref_serialize_tuple(10, attrs, vals, lens, (C.c_uint8 * 10)(), 1 if form == "ref-heap" else 0,
+                                          tw.SENDER_CHUNK_SIZES[seg], buf, 4096, C.byref(nch))
+                parts.append(bytes(buf[:t]))
+            out["senders"][form].append(b"".join(parts).hex())
+    ex._lib = old
+    json.dump(out, open(os.path.join(HERE, "wire_kat.json"), "w"), indent=1)
+    print("wire_kat.json", {k: len(v["stream"]) // 2 for k, v in out["partial"].items()})
+
+
 if __name__ == "__main__":
     R.ref_last_error.restype = C.c_char_p
     if len(sys.argv) > 1:                  # only the named fixtures: python make_golden.py memtuple_kat
@@ -689,3 +778,6 @@ if __name__ == "__main__":
     memtuple_kat()
     numeric_kat()
     mvcc_kat()
+    hash_random_kat()
+    aocs_random_kat()
+    wire_kat()

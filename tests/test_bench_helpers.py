@@ -68,6 +68,7 @@ def test_a_failing_rjoin_child_costs_the_entry_not_the_run(monkeypatch):
     import types
     monkeypatch.setenv("MASTER_PORT", "29611")
     monkeypatch.setenv("GGB200_RJOIN_TIMEOUT", "120")
+    monkeypatch.setenv("CUDA_VISIBLE_DEVICES", "")          # the child sees no device on a GPU machine either
     t0 = time.time()
     r = bench.rjoin_in_children(types.SimpleNamespace(rjoin_rows=2e6), 0, 1)
     assert "error" in r and "child exited" in r["error"] and time.time() - t0 < 110

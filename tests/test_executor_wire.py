@@ -2,10 +2,10 @@
 chunks (GgExecSendTupleChunks) and the reference's own CvtChunksToTup reads them; rows the reference's SerializeTuple wrote —
 as MemTuples and in the heap-tuple form — arrive at a Motion node (GgExecRecvTupleChunks) and the FINAL stage above it gives the
 one-stage answer.  Host C of the product (gg_executor.c + gg_tupser.c) over the oracle-backed stand-in device library; the
-reference side is oracle/_ref (memtuple.o, tupser.o, tupchunklist.o compiled from /root/reference)."""
+reference side (memtuple.o, tupser.o, tupchunklist.o) ran when tests/golden/wire_kat.json was made (make_golden.py wire_kat):
+the streams it read and what it read from them, and the streams it wrote."""
 import ctypes as C
 import os
-import struct
 import sys
 
 import numpy as np
@@ -18,22 +18,30 @@ sys.path.insert(0, HERE)
 
 from greengage_b200 import capi, executor as ex, tpch  # noqa: E402
 from oracle import pyoracle as po  # noqa: E402
+from _util import golden  # noqa: E402
 from test_executor_multiseg import MockRel, build_mock  # noqa: E402
 
 NSEG = 3
 ROWS = 30_000
+PARTIAL_CHUNK_SIZES = (8124, 64)            # segment 0's PARTIAL rows as this engine's tuple chunks
+SENDER_CHUNK_SIZES = (48, 8124, 8124)       # every segment's rows as the reference's SerializeTuple writes them
 
 
-@pytest.fixture(scope="module")
-def mock(tmp_path_factory):
-    so = build_mock(str(tmp_path_factory.mktemp("mockwire")))
-    L = ex.bind(C.CDLL(so))
+def bind_mock(L):
+    """the executor surface and the tuple-chunk entry points of the mock-linked host code"""
+    L = ex.bind(L)
     L.mock_engine.restype = C.c_void_p
     L.mock_relation.restype = C.c_void_p
     L.mock_relation.argtypes = [C.c_void_p, C.c_uint64]
     L.GgExecSendTupleChunks.restype = C.c_int64
     L.GgExecSendTupleChunks.argtypes = [C.c_void_p, C.c_int, C.c_void_p, C.c_uint64, C.POINTER(C.c_int64)]
     L.GgExecRecvTupleChunks.argtypes = [C.c_void_p, C.c_void_p, C.c_uint64]
+    return L
+
+
+@pytest.fixture(scope="module")
+def mock(tmp_path_factory):
+    L = bind_mock(C.CDLL(build_mock(str(tmp_path_factory.mktemp("mockwire")))))
     old = ex._lib
     ex._lib = L
     yield L
@@ -60,79 +68,35 @@ def partial_chunks(L, eng, seg, max_chunk):
     return bytes(out[:got]), n.value, rows
 
 
-WIRE = [(1042, -1, 'i', 0), (1042, -1, 'i', 0)] + [(701, 8, 'd', 1)] * 4 + [(1022, -1, 'd', 0)] * 3 + [(20, 8, 'd', 1)]
-
-
-def wire_attrs():
-    a = (capi.gg_attr * len(WIRE))()
-    for i, (t, l, al, bv) in enumerate(WIRE):
-        a[i].atttypid, a[i].attlen, a[i].attalign, a[i].attbyval, a[i].atttypmod = t, l, ord(al), bv, -1
-    return a
-
-
 def b2f(v):
     return np.int64(v).view(np.float64).item()
 
 
 def test_partial_rows_leave_as_the_references_chunks_and_its_reader_reads_them(mock):
-    R = po.ref_lib()
-    if R is None:
-        pytest.skip("oracle/_ref is not built")
+    """the stream is byte for byte the one the reference's CvtChunksToTup read, and what it read is these rows"""
+    kat = golden("wire_kat.json")["partial"]
     eng = mock.mock_engine()
-    attrs = wire_attrs()
-    for max_chunk in (8124, 64):
+    for max_chunk in PARTIAL_CHUNK_SIZES:
         stream, n, rows = partial_chunks(mock, eng, 0, max_chunk)
         assert n == len(rows) == 4 and stream[-4:] == b"\x00\x00\x04\x00"          # ends with TC_END_OF_STREAM
-        pos = 0
-        for v, nl, ty, ln in rows:
-            # one tuple's chunks: up to and including the WHOLE / PARTIAL_END chunk
-            end = pos
-            while True:
-                size, typ = struct.unpack_from("<HH", stream, end)
-                end += 4 + size
-                if typ in (0, 3):
-                    break
-            vals, lens, nulls, sb = (C.c_int64 * 10)(), (C.c_int32 * 10)(), (C.c_uint8 * 10)(), (C.c_uint8 * 1024)()
-            assert R.ref_deserialize_tuple(10, attrs, stream[pos:end], end - pos, vals, lens, nulls, sb, 1024) == 1       # a MemTuple
-            sbb = bytes(sb)
-            assert sbb[vals[0]:vals[0] + lens[0]] == capi.unpack_str(v[0], ln[0]).encode()
-            assert sbb[vals[1]:vals[1] + lens[1]] == capi.unpack_str(v[1], ln[1]).encode()
-            for k in range(4):
-                assert vals[2 + k] == v[2 + k]                                   # float8 sums: the same bits
+        assert stream.hex() == kat[str(max_chunk)]["stream"], max_chunk
+        for (v, nl, ty, ln), got in zip(rows, kat[str(max_chunk)]["read"], strict=True):
+            assert got["form"] == 1 and got["nulls"] == [0] * 10                         # a MemTuple
+            assert got["keys"] == [capi.unpack_str(v[0], ln[0]), capi.unpack_str(v[1], ln[1])]
+            assert got["sums"] == v[2:6]                                                   # float8 sums: the same bits
             for k in range(3):
-                arr = struct.unpack_from("<iiIii3d", sbb, vals[6 + k])
-                assert arr[:5] == (1, 0, 701, 3, 1) and lens[6 + k] == 44
-                assert [np.float64(x).view(np.int64).item() for x in arr[5:]] == list(v[6 + 3 * k:9 + 3 * k])
-            assert vals[9] == v[15]
-            pos = end
-        assert pos == len(stream) - 4
+                assert got["arrays"][k] == [1, 0, 701, 3, 1] + v[6 + 3 * k:9 + 3 * k] and got["array_lens"][k] == 44
+            assert got["count"] == v[15]
 
 
 @pytest.mark.parametrize("form", ["ours", "ref-memtuple", "ref-heap"])
 def test_rows_from_cpu_senders_arrive_at_the_motion_and_the_final_stage_combines_them(mock, form):
-    R = po.ref_lib()
-    if form != "ours" and R is None:
-        pytest.skip("oracle/_ref is not built")
     eng = mock.mock_engine()
-    attrs = wire_attrs()
-    streams = []
-    for seg in range(NSEG):
-        stream, n, rows = partial_chunks(mock, eng, seg, 8124 if seg else 80)
-        if form == "ours":
-            streams.append(stream[:-4])
-            continue
-        # the same rows written by the reference's SerializeTuple
-        parts = []
-        for v, nl, ty, ln in rows:
-            keep = [C.create_string_buffer(capi.unpack_str(v[k], ln[k]).encode(), max(ln[k], 1)) for k in range(2)]
-            arrs = [C.create_string_buffer(struct.pack("<iiIii3d", 1, 0, 701, 3, 1, *[b2f(x) for x in v[6 + 3 * k:9 + 3 * k]]), 44) for k in range(3)]
-            vals = (C.c_int64 * 10)(C.addressof(keep[0]), C.addressof(keep[1]), v[2], v[3], v[4], v[5], C.addressof(arrs[0]), C.addressof(arrs[1]), C.addressof(arrs[2]), v[15])
-            lens = (C.c_int32 * 10)(ln[0], ln[1], 0, 0, 0, 0, 44, 44, 44, 0)
-            nulls = (C.c_uint8 * 10)()
-            out, nch = (C.c_uint8 * 4096)(), C.c_int32(0)
-            t = R.ref_serialize_tuple(10, attrs, vals, lens, nulls, 1 if form == "ref-heap" else 0, 8124 if seg else 48, out, 4096, C.byref(nch))
-            parts.append(bytes(out[:t]))
-        streams.append(b"".join(parts))
+    if form == "ours":
+        streams = [partial_chunks(mock, eng, seg, 8124 if seg else 80)[0][:-4] for seg in range(NSEG)]
+    else:
+        streams = [bytes.fromhex(h) for h in golden("wire_kat.json")["senders"][form]]
+        assert len(streams) == NSEG
     wire = b"".join(streams) + b"\x00\x00\x04\x00"
     # the receiving slice: Agg(FINAL) <- Gather Motion <- [Agg(PARTIAL) <- SeqScan on the senders]
     scan, part, pool = tpch.q1_plan(capi.TAB_LINEITEM_WIDE, capi.AGGSTAGE_PARTIAL)

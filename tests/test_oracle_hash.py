@@ -1,9 +1,12 @@
 """The oracle's hashing and segment routing against golden vectors computed by the reference's own
-hashfunc.o / varchar.o / cdbhash.o (tests/golden/make_golden.py), and against those objects directly
-when oracle/_ref/libggref.so is present.  The product's host-side routing (libgghost) is held to the
+hashfunc.o / varchar.o / cdbhash.o (tests/golden/make_golden.py), value by value and, for 20000 random
+inputs, as digests of what those objects returned.  The product's host-side routing (libgghost) is held to the
 same vectors."""
 import ctypes as C
+import hashlib
 import random
+
+import numpy as np
 
 from _util import golden
 from greengage_b200 import capi
@@ -60,21 +63,36 @@ def test_routing_golden_oracle_and_product():
         assert H.gg_cdbhash_route(t, v, ln, nu, n, r["nsegs"]) == r["seg"]
 
 
-def test_against_reference_objects_when_built():
-    R = po.ref_lib()
-    if R is None:
-        import pytest
-        pytest.skip("oracle/_ref not built (no /root/reference on this box); golden vectors cover it")
+RANDOM_CASES = 20000
+
+
+def random_hash_outputs(fn, name):
+    """fn's answers to the RANDOM_CASES inputs random.Random(7) draws, as an array: hash_any of 0..48 random bytes ("hash_any"),
+    hashint8 of a random int8 ("hashint8"), or the segment a random int8 key routes to among 1..999 ("route")."""
     rng = random.Random(7)
-    for _ in range(20000):
+    out = []
+    for _ in range(RANDOM_CASES):
         n = rng.randint(0, 48)
         b = bytes(rng.getrandbits(8) for _ in range(n))
-        assert R.ref_hash_any(b, n) == L.or_hash_any(b, n)
         v = rng.getrandbits(64) - (1 << 63)
-        assert R.ref_hashint8(v) == L.or_hashint8(v)
         ns = rng.choice([1, 2, 3, 5, 8, 13, 64, 999])
-        t, vv, ln, nu = (C.c_int32 * 1)(20), (C.c_int64 * 1)(v), (C.c_int32 * 1)(0), (C.c_int32 * 1)(0)
-        assert R.ref_cdbhash_route(t, vv, ln, nu, 1, ns) == L.or_route_datums(t, vv, ln, nu, 1, ns)
+        if name == "hash_any":
+            out.append(fn(b, n))
+        elif name == "hashint8":
+            out.append(fn(v))
+        else:
+            t, vv, ln, nu = (C.c_int32 * 1)(20), (C.c_int64 * 1)(v), (C.c_int32 * 1)(0), (C.c_int32 * 1)(0)
+            out.append(fn(t, vv, ln, nu, 1, ns))
+    return np.array(out, dtype=np.int32 if name == "route" else np.uint32)
+
+
+def test_against_reference_objects_when_built():
+    """The oracle on RANDOM_CASES random inputs against what the reference's own hashfunc.o / cdbhash.o returned for them
+    (tests/golden/hash_random_kat.json keeps a SHA-256 digest of each output sequence; make_golden.py hash_random_kat)."""
+    kat = golden("hash_random_kat.json")
+    assert kat["cases"] == RANDOM_CASES
+    for name, fn in (("hash_any", L.or_hash_any), ("hashint8", L.or_hashint8), ("route", L.or_route_datums)):
+        assert hashlib.sha256(random_hash_outputs(fn, name).tobytes()).hexdigest() == kat[name], name
 
 
 def test_bulk_routing_of_aggregate_rows_matches_the_oracle():
